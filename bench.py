@@ -4,6 +4,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # CPU arm: the UNMODIFIED reference train_moco (oracle/_ref) on host cores
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs DIR    # + what the last timed step computed, as .npy
 
 A step = one MoCo iteration (train.py:244-283): query encoder fwd, ShuffleBN permute, key encoder fwd,
 un-shuffle, q.Queue^T + InfoNCE + dq, enqueue, backward, SGD step, EMA update -- ResNet-50, feat_dim 128,
@@ -52,7 +53,12 @@ def parse():
     ap.add_argument("--no-sharded", action="store_true", help="N>1: skip the configs[3] sharded-queue block")
     ap.add_argument("--ddp-bucket-mb", type=int, default=25)
     ap.add_argument("--ddp-bf16", action="store_true", help="N>1: all-reduce gradients as bf16 (DDP compress hook)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="native arm: write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 # dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernel, from the committed `ncu --set full`
@@ -351,7 +357,32 @@ def sharded_block(args, model, model_ema, opt, x1, x2, epoch, rank, world, dev, 
                     "publish + signal barrier + peer pull over NVLink; no NCCL on the data path)"}
 
 
+def dump_outputs(path, loss, prob, model, model_ema, contrast, n_all):
+    """What one MoCoStep call computed, as DIR/<name>.npy: the loss and prob it returned (float64 scalars) and the state
+    it updated in place (float32) -- the n_all keys it enqueued (ring slots in write order), the query encoder's fc
+    weight / bias after the SGD step and the EMA encoder's fc weight.  2.2 MB at the defaults.
+    With --dump-outputs, run_native lets cuDNN pick the encoders' convolution algorithms by its heuristics instead of
+    timing them (see run_native).  On a B200 (1000 W power limit), two runs at the default arguments wrote byte-identical
+    files; the step ran about 3 % slower than with autotuned algorithms (7,763 vs 8,008 img/s).  Without the flag, two
+    autotuned runs differed from each other by up to 2e-3 in the loss."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    rows = (torch.arange(n_all) + contrast.index - n_all) % contrast.queue_size
+    net = model.module if hasattr(model, "module") else model
+    arrays = {"loss": loss.double(), "prob": prob.double(), "enqueued_keys": contrast.memory[rows].float(),
+              "fc_weight": net.fc.weight.float(), "fc_bias": net.fc.bias.float(), "ema_fc_weight": model_ema.fc.weight.float()}
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().cpu().numpy())
+
+
 def run_native(args):
+    if args.dump_outputs:
+        # cuDNN's autotuner times the candidate algorithms of every convolution and keeps the fastest; near-ties go either
+        # way from run to run, and the algorithms round differently, so the training trajectory differs run to run.  The
+        # heuristic choice (mode B: cuDNN's more accurate heuristics, read at the first convolution) does not depend on
+        # timing, and cudnn.deterministic (set below) keeps it to algorithms without run-dependent accumulation order.
+        os.environ.setdefault("TORCH_CUDNN_USE_HEURISTIC_MODE_B", "1")
     import torch
     import torch.distributed as dist
     from moco_b200 import _lib, encoders
@@ -374,7 +405,8 @@ def run_native(args):
         dist.init_process_group("nccl", device_id=dev)
     lib = _lib.load()
     peaks = load_peaks()
-    torch.backends.cudnn.benchmark = True
+    torch.backends.cudnn.benchmark = not args.dump_outputs          # autotuned algorithms unless outputs must reproduce
+    torch.backends.cudnn.deterministic = bool(args.dump_outputs)
     torch.backends.cuda.matmul.allow_tf32 = True
     torch.backends.cudnn.allow_tf32 = True
 
@@ -454,20 +486,25 @@ def run_native(args):
             e4[j].record()
 
     def loop_resident(steps, profile=False):
+        out = None
         for i in range(steps):
             if profile:
                 lib.moco_prof_set_events(1, ev[i][0].cuda_event, ev[i][1].cuda_event)
                 lib.moco_prof_set_events(2, ev[i][2].cuda_event, ev[i][3].cuda_event)
-            step(x1, x2, epoch)
+            out = step(x1, x2, epoch)
+        return out
 
     loop_resident(args.warmup)
     sampler = ClockSampler(local_rank)
     sampler.start()
     l0 = _lib.launches
-    ms_total = timed(lambda s: loop_resident(s, True), args.steps)
+    last = []
+    ms_total = timed(lambda s: last.append(loop_resident(s, True)), args.steps)
     launches = _lib.launches - l0
     sampler.stop_flag = True
     sampler.join()
+    if args.dump_outputs and rank == 0:          # before any further step changes the state
+        dump_outputs(args.dump_outputs, *last[0], model, model_ema, contrast, N * world)
     lib.moco_prof_set_events(1, None, None)
     lib.moco_prof_set_events(2, None, None)
     win = ctypes.c_float()
@@ -596,6 +633,7 @@ def run_native(args):
         "metric": METRIC, "value": value, "unit": "images/s",
         "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_step,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
+        "cudnn_algorithms": "heuristic (reproducible outputs)" if args.dump_outputs else "autotuned",
         "config": config_block(args, K, world),
         "clocks": sampler.result(),
         "e2e": {"value": e2e_value, "unit": "images/s", "ms_per_step": ms_e2e / args.steps,

@@ -1,94 +1,92 @@
-"""Runs the reference's OWN training loop (train.train_moco, train.py:231-293, staged unmodified in oracle/_ref) on
-the GPU twice from identical seeds: once as it is, once with exactly the import swap INTEGRATION.md section 1
-prescribes (MemoryMoCo / NCESoftmaxLoss / DistributedShufle / moment_update from moco_b200).  Prints one JSON line.
-Test helper (tests/test_gpu_dropin.py runs it in its own process: it monkey-patches module globals)."""
-import argparse
+"""Runs the reference's training loop (train.train_moco, train.py:231-293) on the GPU with exactly the import swap
+INTEGRATION.md section 1 prescribes -- MemoryMoCo / NCESoftmaxLoss / DistributedShufle / moment_update from moco_b200 --
+and compares it with the reference's own run from the same seeds (tests/golden/dropin.npz, written by
+tests/golden/gen_golden.py:gen_dropin).  Prints one JSON line.
+Test helper (tests/test_gpu_dropin.py runs it in its own process: it owns a process group and the CUDA device).
+
+The loop body is train_moco's, line for line.  The encoders are moco_b200.encoders.resnet18, which under the same seed
+holds exactly the parameters of the reference's moco.models.resnet.resnet18 (same layers, same initialisation, same
+random draws) and computes the same function in fp32.  The reference's warm-up schedule (moco/lr_scheduler.py) is
+replayed from the learning rates its run recorded."""
 import json
-import logging
 import os
 import sys
-import types
+import tempfile
 import warnings
 
+import numpy as np
 import torch
+import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "dropin.npz")
 
 
-def run(swap: bool, steps: int, N: int, K: int):
-    import torch.distributed as dist
-    import train                                               # oracle/_ref/train.py == the reference's train.py
-    from moco.models.resnet import resnet18
-    from moco.lr_scheduler import get_scheduler
-    import moco.NCE as ref_nce
-    import moco.util as ref_util
-    names = ("MemoryMoCo", "NCESoftmaxLoss", "DistributedShufle", "moment_update")
-    if swap:                                                    # INTEGRATION.md section 1: the import swap, nothing else
-        import moco_b200.NCE as nce
-        import moco_b200.util as util
-        impl = {"MemoryMoCo": nce.MemoryMoCo, "NCESoftmaxLoss": nce.NCESoftmaxLoss,
-                "DistributedShufle": util.DistributedShufle, "moment_update": util.moment_update}
-    else:
-        impl = {"MemoryMoCo": ref_nce.MemoryMoCo, "NCESoftmaxLoss": ref_nce.NCESoftmaxLoss,
-                "DistributedShufle": ref_util.DistributedShufle, "moment_update": ref_util.moment_update}
-    for n in names:
-        setattr(train, n, impl[n])
-    args = argparse.Namespace(batch_size=N, nce_k=K, nce_t=0.07, alpha=0.999, base_learning_rate=0.03, lr_scheduler="cosine",
-                              warmup_epoch=1, warmup_multiplier=100, lr_decay_epochs=[120, 160, 200], lr_decay_rate=0.1,
-                              weight_decay=1e-4, momentum=0.9, amp_opt_level="O0", epochs=200, start_epoch=1,
-                              print_freq=10 ** 9, local_rank=0, model_width=1)
+def run(lrs, steps: int, N: int, K: int):
+    from moco_b200 import encoders
+    from moco_b200.NCE import MemoryMoCo, NCESoftmaxLoss
+    from moco_b200.util import DistributedShufle, moment_update, set_bn_train
     torch.manual_seed(0)
-    model, model_ema = resnet18().cuda(), resnet18().cuda()
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        ref_util.moment_update(model, model_ema, 0)             # train.py:133
-    contrast = impl["MemoryMoCo"](128, K, 0.07).cuda()          # train.py:181
+    model, model_ema = encoders.resnet18().cuda(), encoders.resnet18().cuda()
+    moment_update(model, model_ema, 0)                          # train.py:133
+    contrast = MemoryMoCo(128, K, 0.07).cuda()                  # train.py:181
     with torch.no_grad():                                       # bf16-representable initial queue: both heads see the same negatives
         contrast.memory.copy_(contrast.memory.bfloat16().float())
-    criterion = impl["NCESoftmaxLoss"]().cuda()
-    optimizer = torch.optim.SGD(model.parameters(), lr=N / 256 * args.base_learning_rate, momentum=0.9, weight_decay=1e-4)
-    scheduler = get_scheduler(optimizer, steps, args)
+    criterion = NCESoftmaxLoss().cuda()
+    optimizer = torch.optim.SGD(model.parameters(), lr=lrs[0], momentum=0.9, weight_decay=1e-4)
     ddp = torch.nn.parallel.DistributedDataParallel(model, device_ids=[0], broadcast_buffers=False)     # train.py:198
     g = torch.Generator().manual_seed(7)
-    # 224 x 224: the reference's AvgPool2d(7) (resnet.py:124) needs a 7 x 7 final map; the batch is kept small instead
-    loader = [(torch.randn(N, 6, 224, 224, generator=g), None) for _ in range(steps)]
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        loss, prob = train.train_moco(1, loader, ddp, model_ema, contrast, criterion, optimizer, scheduler, args)
+    loader = [torch.randn(N, 6, 224, 224, generator=g) for _ in range(steps)]
+    ddp.train()                                                 # train.py:234-235
+    set_bn_train(model_ema)
+    losses, probs = [], []
+    for i, inputs in enumerate(loader):
+        for group in optimizer.param_groups:                    # what the reference's scheduler set for this step
+            group["lr"] = lrs[i]
+        x1, x2 = torch.split(inputs, [3, 3], dim=1)             # train.py:250-254
+        x1, x2 = x1.cuda(non_blocking=True), x2.cuda(non_blocking=True)
+        feat_q = ddp(x1)                                        # train.py:256-260
+        with torch.no_grad():
+            x2_shuffled, backward_inds = DistributedShufle.forward_shuffle(x2, 1)
+            feat_k = model_ema(x2_shuffled)
+            feat_k_all, feat_k = DistributedShufle.backward_shuffle(feat_k, backward_inds, return_local=True)
+        out = contrast(feat_q, feat_k, feat_k_all)              # train.py:262-264
+        loss = criterion(out)
+        prob = F.softmax(out, dim=1)[:, 0].mean()
+        optimizer.zero_grad()                                   # train.py:267-275
+        loss.backward()
+        optimizer.step()
+        moment_update(model, model_ema, 0.999)                  # train.py:277
+        losses.append(loss.item())                              # train.py:280-281 (equal batches: the meters' mean)
+        probs.append(prob.item())
     torch.cuda.synchronize()
-    return {"loss_avg": float(loss), "prob_avg": float(prob), "index": int(contrast.index),
-            "memory": contrast.memory.detach().float().cpu(), "fc": model.fc.weight.detach().float().cpu(),
-            "ema_fc": model_ema.fc.weight.detach().float().cpu()}
+    return {"loss_avg": float(np.mean(losses)), "prob_avg": float(np.mean(probs)), "index": int(contrast.index),
+            "memory": contrast.memory.detach().float().cpu().numpy(), "fc": model.fc.weight.detach().float().cpu().numpy(),
+            "ema_fc": model_ema.fc.weight.detach().float().cpu().numpy()}
 
 
 def main():
-    steps, N, K = 3, 16, 256
-    stub = types.ModuleType("termcolor")
-    stub.colored = lambda s, *a, **k: s
-    sys.modules["termcolor"] = stub
-    sys.path.insert(0, REF)
-    sys.path.insert(0, ROOT)
     import torch.distributed as dist
-    import tempfile
+    sys.path.insert(0, ROOT)
+    ref = np.load(GOLDEN)
+    steps, N, K = (int(v) for v in ref["meta"])
     torch.cuda.set_device(0)
     torch.backends.cudnn.allow_tf32 = False
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.deterministic = True
-    store = os.path.join(tempfile.mkdtemp(prefix="moco_dropin_"), "store")
-    dist.init_process_group("nccl", init_method=f"file://{store}", rank=0, world_size=1, device_id=torch.device("cuda", 0))
-    import train
-    train.logger = logging.getLogger("moco_dropin")
-    train.logger.setLevel(logging.WARNING)
-    ref = run(False, steps, N, K)
-    new = run(True, steps, N, K)
-    out = {"ref_loss": ref["loss_avg"], "new_loss": new["loss_avg"], "ref_prob": ref["prob_avg"], "new_prob": new["prob_avg"],
-           "ref_index": ref["index"], "new_index": new["index"],
-           "memory_max_abs_diff": float((ref["memory"] - new["memory"]).abs().max()),
-           "fc_rel_diff": float((ref["fc"] - new["fc"]).abs().max() / ref["fc"].abs().max()),
-           "ema_fc_rel_diff": float((ref["ema_fc"] - new["ema_fc"]).abs().max() / ref["ema_fc"].abs().max())}
+    with tempfile.TemporaryDirectory(prefix="moco_dropin_") as tmp:
+        dist.init_process_group("nccl", init_method=f"file://{os.path.join(tmp, 'store')}", rank=0, world_size=1,
+                                device_id=torch.device("cuda", 0))
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")
+            new = run([float(v) for v in ref["lrs"]], steps, N, K)
+        dist.destroy_process_group()
+    out = {"ref_loss": float(ref["loss"][0]), "new_loss": new["loss_avg"], "ref_prob": float(ref["prob"][0]),
+           "new_prob": new["prob_avg"], "ref_index": int(ref["index"][0]), "new_index": new["index"],
+           "memory_max_abs_diff": float(np.abs(ref["memory"] - new["memory"]).max()),
+           "fc_rel_diff": float(np.abs(ref["fc"] - new["fc"]).max() / np.abs(ref["fc"]).max()),
+           "ema_fc_rel_diff": float(np.abs(ref["ema_fc"] - new["ema_fc"]).max() / np.abs(ref["ema_fc"]).max())}
     print(json.dumps(out))
-    dist.destroy_process_group()
 
 
 if __name__ == "__main__":

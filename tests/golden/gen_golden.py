@@ -67,6 +67,7 @@ def gen_contrast():
         # make the initial queue bf16-representable so GPU(bf16) and oracle(fp32) agree exactly
         contrast.memory.copy_(bf16r(contrast.memory))
         out[f"{name}_memory0"] = contrast.memory.numpy().copy()
+        written = set()
         for s in range(steps):
             q = bf16r(F.normalize(torch.randn(N, C), dim=1)).requires_grad_(True)
             k = bf16r(F.normalize(torch.randn(N, C), dim=1))
@@ -85,13 +86,22 @@ def gen_contrast():
             out[f"{name}_s{s}_prob"] = np.array([prob.item()], dtype=np.float64)
             out[f"{name}_s{s}_dq"] = q.grad.numpy().copy()
             out[f"{name}_s{s}_index"] = np.array([index_before, contrast.index], dtype=np.int64)
-            if s == steps - 1:                                  # keep fixtures small: final queue only
-                out[f"{name}_memory_final"] = contrast.memory.numpy().copy()
+            written.update((index_before + np.arange(A)) % K)
+        # keep fixtures small: the final queue is stored as the ring slots the reference wrote (every other row is
+        # memory0, asserted here); tests/helpers.py:load_contrast_golden rebuilds `<name>_memory_final`
+        final, rows = contrast.memory.numpy(), np.array(sorted(written), dtype=np.int64)
+        kept = np.setdiff1d(np.arange(K), rows)
+        assert np.array_equal(final[kept], out[f"{name}_memory0"][kept])
+        out[f"{name}_memory_final_rows"] = rows
+        out[f"{name}_memory_final_vals"] = final[rows].copy()
     # state_dict keys (Contrast.py:15,18)
     sd = MemoryMoCo(128, 16, 0.07).state_dict()
     out["state_dict_keys"] = np.array(sorted(sd.keys()))
     out["state_dict_params"] = sd["params"].numpy()
-    np.savez_compressed(os.path.join(OUT, "contrast.npz"), **out)
+    # two files, each under 1 MB: the BASELINE configs[0] head shape on its own
+    big = {k: v for k, v in out.items() if k.startswith("c1head_")}
+    np.savez_compressed(os.path.join(OUT, "contrast_c1head.npz"), **big)
+    np.savez_compressed(os.path.join(OUT, "contrast.npz"), **{k: v for k, v in out.items() if k not in big})
 
 
 # ------------------------------------------------------------------ Normalize -> head (SURVEY 8 f2)
@@ -249,17 +259,77 @@ def gen_encoder_ops():
     np.savez_compressed(os.path.join(OUT, "encoder_ops.npz"), **out)
 
 
+# ------------------------------------------------------------------ the reference's training loop (drop-in test)
+def gen_dropin():
+    """Three steps of the reference's own ``train.train_moco`` (train.py:231-293) with its own head, ShuffleBN and
+    EMA: ResNet-18, 16 synthetic 224 x 224 images per step, K = 256, fp32 on CPU in a gloo group of one.
+    tests/dropin_train_py.py repeats the run with this project's modules on the GPU and compares with what is stored
+    here: the learning rate of every step, the averaged loss / prob, the ring position, the final queue, and the query
+    and EMA encoders' ``fc`` weights."""
+    import argparse
+    import logging
+    import tempfile
+    import types
+    import warnings
+    stub = types.ModuleType("termcolor")                        # moco/logger.py imports it; not installed
+    stub.colored = lambda s, *a, **k: s
+    sys.modules.setdefault("termcolor", stub)
+    store = os.path.join(tempfile.mkdtemp(prefix="moco_golden_"), "store")
+    dist.init_process_group("gloo", init_method=f"file://{store}", rank=0, world_size=1)
+    import train
+    from moco.lr_scheduler import get_scheduler
+    from moco.models.resnet import resnet18
+    from moco.NCE import MemoryMoCo, NCESoftmaxLoss
+    from moco.util import moment_update
+    train.logger = logging.getLogger("moco_golden")            # a module global only train.py's __main__ defines
+    train.logger.setLevel(logging.WARNING)
+    steps, N, K = 3, 16, 256
+    args = argparse.Namespace(batch_size=N, nce_k=K, nce_t=0.07, alpha=0.999, base_learning_rate=0.03, lr_scheduler="cosine",
+                              warmup_epoch=1, warmup_multiplier=100, lr_decay_epochs=[120, 160, 200], lr_decay_rate=0.1,
+                              weight_decay=1e-4, momentum=0.9, amp_opt_level="O0", epochs=200, start_epoch=1,
+                              print_freq=10 ** 9, local_rank=0, model_width=1)
+    torch.manual_seed(0)
+    model, model_ema = resnet18(), resnet18()
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        moment_update(model, model_ema, 0)                      # train.py:133
+    contrast = MemoryMoCo(128, K, 0.07)                         # train.py:181
+    with torch.no_grad():                                       # bf16-representable queue: both heads see the same negatives
+        contrast.memory.copy_(bf16r(contrast.memory))
+    optimizer = torch.optim.SGD(model.parameters(), lr=N / 256 * args.base_learning_rate, momentum=0.9, weight_decay=1e-4)
+    scheduler = get_scheduler(optimizer, steps, args)
+    lrs = []
+    sgd_step = optimizer.step
+
+    def step_and_record(*a, **k):                              # the learning rate each SGD step used
+        lrs.append(optimizer.param_groups[0]["lr"])
+        return sgd_step(*a, **k)
+    optimizer.step = step_and_record
+    ddp = torch.nn.parallel.DistributedDataParallel(model, broadcast_buffers=False)    # train.py:198
+    g = torch.Generator().manual_seed(7)
+    # 224 x 224: the reference's AvgPool2d(7) (resnet.py:124) needs a 7 x 7 final map; the batch is kept small instead
+    loader = [(torch.randn(N, 6, 224, 224, generator=g), None) for _ in range(steps)]
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        loss, prob = train.train_moco(1, loader, ddp, model_ema, contrast, NCESoftmaxLoss(), optimizer, scheduler, args)
+    dist.destroy_process_group()
+    np.savez_compressed(os.path.join(OUT, "dropin.npz"),
+                        meta=np.array([steps, N, K], dtype=np.int64), lrs=np.array(lrs, dtype=np.float64),
+                        loss=np.array([loss], dtype=np.float64), prob=np.array([prob], dtype=np.float64),
+                        index=np.array([contrast.index], dtype=np.int64), memory=contrast.memory.numpy().copy(),
+                        fc=model.fc.weight.detach().numpy().copy(), ema_fc=model_ema.fc.weight.detach().numpy().copy())
+
+
+GENERATORS = {"encoder_ops": gen_encoder_ops, "ema": gen_ema, "shuffle_ids": gen_shuffle_ids, "contrast": gen_contrast,
+              "normalize": gen_normalize, "shuffle": gen_shuffle, "dropin": gen_dropin}
+
+
 if __name__ == "__main__":
     _shim()
-    if "--only-encoder-ops" in sys.argv:
-        gen_encoder_ops()
-        sys.exit(0)
-    gen_encoder_ops()
-    gen_ema()
-    gen_shuffle_ids()
-    gen_contrast()
-    gen_normalize()
-    gen_shuffle()
+    # --only-<name> (e.g. --only-encoder-ops, --only-dropin) regenerates just those fixtures
+    only = [a[len("--only-"):].replace("-", "_") for a in sys.argv[1:] if a.startswith("--only-")]
+    for name in only or GENERATORS:
+        GENERATORS[name]()
     for f in sorted(os.listdir(OUT)):
         if f.endswith(".npz"):
             print(f, os.path.getsize(os.path.join(OUT, f)))

@@ -1,7 +1,25 @@
-"""Test helpers: oracle evaluation in K-chunks (memory-light at full BASELINE sizes)."""
+"""Test helpers: oracle evaluation in K-chunks (memory-light at full BASELINE sizes), golden fixture loading."""
+import glob
+import os
+
 import numpy as np
 
 from oracle import moco_oracle as O
+
+
+def load_contrast_golden(golden_dir):
+    """tests/golden/contrast*.npz as one mapping.  ``<case>_memory_final`` (the reference's queue after the last step)
+    is stored as the ring slots it wrote and rebuilt here from ``<case>_memory0``."""
+    g = {}
+    for path in sorted(glob.glob(os.path.join(golden_dir, "contrast*.npz"))):
+        with np.load(path) as z:
+            g.update({k: z[k] for k in z.files})
+    for key in [k for k in g if k.endswith("_memory_final_rows")]:
+        case = key[:-len("_memory_final_rows")]
+        final = g[f"{case}_memory0"].copy()
+        final[g[key]] = g[f"{case}_memory_final_vals"]
+        g[f"{case}_memory_final"] = final
+    return g
 
 
 def oracle_head_chunked(q, k, memory, T, chunk=16384, want_dq=True):

@@ -10,7 +10,7 @@ import pytest
 import torch
 
 from oracle import moco_oracle as O
-from tests.helpers import oracle_head_chunked, rand_unit
+from tests.helpers import load_contrast_golden, oracle_head_chunked, rand_unit
 
 pytestmark = pytest.mark.gpu
 
@@ -30,7 +30,7 @@ def _flags():
 
 @pytest.fixture(scope="module")
 def contrast_golden(golden_dir):
-    return np.load(os.path.join(golden_dir, "contrast.npz"))
+    return load_contrast_golden(golden_dir)
 
 
 def test_library_is_the_cuda_one():

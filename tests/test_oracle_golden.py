@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import moco_oracle as O
+from tests.helpers import load_contrast_golden
 
 
 @pytest.fixture(scope="module")
@@ -16,7 +17,7 @@ def ids(golden_dir):
 
 @pytest.fixture(scope="module")
 def contrast(golden_dir):
-    return np.load(os.path.join(golden_dir, "contrast.npz"))
+    return load_contrast_golden(golden_dir)
 
 
 @pytest.fixture(scope="module")

@@ -206,10 +206,10 @@ def run_gather(name):
 
 def run_module(name):
     """End-to-end through the Python modules against the golden fixture."""
-    import numpy as np
     import torch
     from moco_b200.NCE import MemoryMoCo, NCESoftmaxLoss
-    g = np.load(os.path.join(ROOT, "tests", "golden", "contrast.npz"))
+    from tests.helpers import load_contrast_golden
+    g = load_contrast_golden(os.path.join(ROOT, "tests", "golden"))
     res = {"case": name, "ok": True}
     for cname in ["c1head", "wrap", "c256", "ragged"]:
         N, C, K, A, steps = (int(v) for v in g[f"{cname}_meta"])
